@@ -16,6 +16,10 @@ Before the timed region every rank set runs (untimed, `--no-verify` skips it):
 
 `--impl reference` times the CPU restatement of the reference path (the oracle; the real lightgbmlib
 3.2.110 cannot be built or installed here — BASELINE.md §2) on a bounded row sample of the same workload.
+
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step computed as float64 .npy files (see
+dump_outputs()).  The workload is synthesised from fixed seeds, so two builds run with the same arguments can be
+compared output for output.
 """
 import argparse
 import hashlib
@@ -442,6 +446,36 @@ def verify_full_size(capi, cfg, ds, n_local, F, row_start, chunk):
     return out
 
 
+DUMP_TREE_KEYS = ("num_leaves", "num_cat", "split_feature", "split_gain", "threshold", "decision_type", "left_child", "right_child",
+                  "leaf_value", "leaf_weight", "leaf_count", "internal_value", "internal_weight", "internal_count", "cat_boundaries",
+                  "cat_threshold")
+DUMP_MAX_SCORES = 4 << 20         # float64 training scores kept in the dump: 32 MB
+
+
+def dump_outputs(out_dir, bst, model_text):
+    """What a caller of LGBM_BoosterUpdateOneIter has after the last timed step, as float64 arrays:
+      tree_<key>.npy     the tree(s) that step added (one per class), read back through the model text; each key of the K trees
+                         concatenated in class order (num_leaves and num_cat say where one tree ends); a key none of the trees
+                         has values for (cat_* without categorical splits, split fields of single-leaf trees) is not written;
+      train_score.npy    the raw training scores after that step, [K][m] for a fixed, seeded sample of m of this rank's rows
+                         (all rows when they fit in DUMP_MAX_SCORES values)."""
+    from mmlspark_b200.modeltext import parse_model
+    os.makedirs(out_dir, exist_ok=True)
+    model = parse_model(model_text)
+    K = int(model["header"]["num_tree_per_iteration"])
+    last = model["trees"][-K:]
+    for key in DUMP_TREE_KEYS:
+        arr = np.concatenate([np.atleast_1d(np.asarray(t.get(key, []), dtype=np.float64)) for t in last])
+        if arr.size:
+            np.save(os.path.join(out_dir, "tree_%s.npy" % key), arr)
+    scores = bst.get_scores(0).reshape(K, -1)
+    n = scores.shape[1]
+    if n * K > DUMP_MAX_SCORES:
+        rows = np.sort(np.random.default_rng(0).choice(n, size=DUMP_MAX_SCORES // K, replace=False))
+        scores = scores[:, rows]
+    np.save(os.path.join(out_dir, "train_score.npy"), np.ascontiguousarray(scores))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -455,7 +489,11 @@ def main():
     ap.add_argument("--cpu-sample-rows", type=int, default=2_000_000)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-verify", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's tree(s) and a sample of the training scores to DIR as .npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -564,6 +602,8 @@ def main():
         if world > 1:
             capi.network_free()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, bst, model_text)
     checks["timed_model"] = {"trees": len(leaves), "min_leaves": min(leaves) if leaves else 0, "hash": mhash,
                              "identical_on_all_ranks": len(set(hashes)) == 1}
     steps = args.steps
