@@ -1,6 +1,7 @@
 // b200gbm engine implementation: network bootstrap, dataset ingestion/binning, GBDT driver and the
 // device-resident leaf-wise tree learner.  See engine.h / kernels.cuh / hist_kernel.cuh.
 #include "engine.h"
+#include "objective.cuh"
 #include "renew_kernel.cuh"
 #include "metric_kernels.cuh"
 
@@ -177,7 +178,7 @@ void NetworkFree() {
 }
 
 // small host-value collectives (init scores, label statistics, bin mappers): stage through device memory
-static void AllReduceHost(double* v, int n, ncclRedOp_t op, cudaStream_t s) {
+void AllReduceHost(double* v, int n, ncclRedOp_t op, cudaStream_t s) {
   if (!Net().active) return;
   DevBuf<double> d; d.Alloc(n);
   d.Upload(v, n, s);
@@ -857,43 +858,7 @@ void Dataset::SetFeatureNames(const char** names, int n) {
   }
 }
 
-// ---- host percentiles for the init score of regression_l1 / quantile / mape
-// [LightGBM regression_objective.hpp PercentileFun / WeightedPercentileFun, T = label_t]: the alpha percentile counted from the
-// top of the descending order d[]: fp = (cnt-1)(1-alpha), interpolation between d[int(fp)] and d[int(fp)+1]; weighted: upper_bound on
-// the running weight sum.
-static float LabelPercentile(const float* y, int cnt, double alpha) {
-  if (cnt <= 1) return y[0];
-  const double float_pos = static_cast<double>(cnt - 1) * (1.0 - alpha);
-  const int pos = static_cast<int>(float_pos) + 1;
-  if (pos < 1) return *std::max_element(y, y + cnt);
-  if (pos >= cnt) return *std::min_element(y, y + cnt);
-  std::vector<float> v(y, y + cnt);
-  std::nth_element(v.begin(), v.begin() + pos, v.end(), std::greater<float>());      // v[pos] = (pos+1)-th largest, larger ones before it
-  const float v2 = v[pos], v1 = *std::min_element(v.begin(), v.begin() + pos);
-  return static_cast<float>(v1 - (v1 - v2) * (float_pos - (pos - 1)));
-}
-static float LabelWeightedPercentile(const float* y, const float* w, int cnt, double alpha) {
-  if (cnt <= 1) return y[0];
-  std::vector<int> order(cnt);
-  std::iota(order.begin(), order.end(), 0);
-  std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return y[a] < y[b]; });
-  std::vector<double> cdf(cnt);
-  cdf[0] = w[order[0]];
-  for (int i = 1; i < cnt; ++i) cdf[i] = cdf[i - 1] + w[order[i]];
-  const double threshold = cdf[cnt - 1] * alpha;
-  size_t pos = std::upper_bound(cdf.begin(), cdf.end(), threshold) - cdf.begin();
-  pos = std::min(pos, static_cast<size_t>(cnt - 1));
-  if (pos == 0 || pos == static_cast<size_t>(cnt - 1)) return y[order[pos]];
-  const float v1 = y[order[pos - 1]], v2 = y[order[pos]];
-  if (cdf[pos + 1] - cdf[pos] >= 1.0f) return static_cast<float>((threshold - cdf[pos]) / (cdf[pos + 1] - cdf[pos]) * (v2 - v1) + v1);
-  return v2;
-}
-
 // =============================================================================== booster
-// dynamic shared memory of k_grad_lambdarank: per-document arrays + the pair matrix of one j-tile
-static size_t LambdarankSmem(int max_q, int truncation) {
-  return static_cast<size_t>(max_q) * (8 + 8 + 4 + 4 + 4 + 4) + 8 + static_cast<size_t>(truncation) * (lr_tile(truncation) + 1) * 8;
-}
 static size_t Align16(size_t x) { return (x + 15) & ~static_cast<size_t>(15); }
 constexpr int kScanSmem = (768 + 64) * 8;         // k_scan: scratch of the categorical split search (one warp per block runs it)
 
@@ -912,20 +877,8 @@ Booster::Booster(const Dataset* tr, const char* params) : train(tr) {
     Fatal("Unknown boosting type " + cfg.boosting);
   is_rf_ = cfg.boosting == "rf"; is_goss_ = cfg.boosting == "goss"; is_dart_ = cfg.boosting == "dart";
   drop_rand_ = LcgRandom(cfg.drop_seed);
-  {
-    static const char* kRegVar[] = {"", "huber", "fair", "poisson", "gamma", "tweedie"};
-    for (int k = 1; k <= 5; ++k) if (cfg.objective == kRegVar[k]) regvar_kind_ = k;
-  }
-  if (cfg.objective == "regression_l1") renew_kind_ = 1;
-  else if (cfg.objective == "quantile") renew_kind_ = 2;
-  else if (cfg.objective == "mape") renew_kind_ = 3;
-  if (renew_kind_ == 2 && !(cfg.alpha > 0.0 && cfg.alpha < 1.0)) Fatal("Check failed: alpha_ > 0 && alpha_ < 1");
-  renew_alpha_ = renew_kind_ == 2 ? static_cast<double>(static_cast<float>(cfg.alpha)) : 0.5;     // quantile keeps alpha as score_t
-  is_ova_ = cfg.objective == "multiclassova";
-  if (cfg.objective != "regression" && cfg.objective != "binary" && cfg.objective != "multiclass" && cfg.objective != "lambdarank" && !is_ova_ &&
-      cfg.objective != "cross_entropy" && !regvar_kind_ && !renew_kind_)
-    Fatal("Unknown/unsupported objective type name: " + cfg.objective);
-  balanced_bagging_ = cfg.bagging_freq > 0 && (cfg.pos_bagging_fraction < 1.0 || cfg.neg_bagging_fraction < 1.0) && cfg.objective == "binary";
+  obj_.reset(new Objective(cfg, train));
+  balanced_bagging_ = cfg.bagging_freq > 0 && (cfg.pos_bagging_fraction < 1.0 || cfg.neg_bagging_fraction < 1.0) && obj_->IsBinary();
   bagging_ = cfg.bagging_freq > 0 && (cfg.bagging_fraction < 1.0 || balanced_bagging_);
   if (bagging_ && !(cfg.bagging_fraction > 0.0)) Fatal("bagging_fraction should be in (0, 1]");
   if (is_goss_) {      // [LightGBM goss.hpp ResetGoss]
@@ -939,10 +892,8 @@ Booster::Booster(const Dataset* tr, const char* params) : train(tr) {
   }
   if (cfg.num_leaves < 2) Fatal("num_leaves should be >= 2");
   ValidateMetrics();      // an unknown metric must fail LGBM_BoosterCreate, not the first LGBM_BoosterGetEval inside the training loop
-  if (train->label.empty()) Fatal("label should not be empty for training");
-  if ((cfg.objective == "multiclass" || is_ova_) && cfg.num_class < 2) Fatal("Number of classes should be specified and greater than 1 for multiclass training");
-  if (cfg.objective == "lambdarank" && train->query_boundaries.empty()) Fatal("Ranking tasks require query information");
-  K = (cfg.objective == "multiclass" || is_ova_) ? cfg.num_class : 1;
+  obj_->CheckData();
+  K = obj_->NumModelPerIteration();
   parallel_ = Net().active && Net().world > 1;
   cfg.num_machines = parallel_ ? Net().world : 1;
   if (balanced_bagging_) {      // [LightGBM GBDT::ResetBaggingConfig] needs (globally) at least one positive row
@@ -964,7 +915,7 @@ Booster::Booster(const Dataset* tr, const char* params) : train(tr) {
   model.feature_names = train->feature_names;
   for (int f = 0; f < train->num_total_features; ++f) model.feature_infos.push_back(train->mappers[f].InfoString());
   InitTraining();
-  model.objective_str = ObjectiveString();
+  model.objective_str = obj_->ToString();
 }
 
 Booster::~Booster() {
@@ -984,11 +935,11 @@ Booster::~Booster() {
   if (stream_) cudaStreamDestroy(stream_);
 }
 
-std::string Booster::ObjectiveString() const {
-  if (cfg.objective == "binary") return "binary sigmoid:" + Config::Num(cfg.sigmoid);
-  if (cfg.objective == "multiclass") return "multiclass num_class:" + std::to_string(cfg.num_class);
-  if (is_ova_) return "multiclassova num_class:" + std::to_string(cfg.num_class) + " sigmoid:" + Config::Num(cfg.sigmoid);
-  return cfg.objective;
+void Booster::GetInfo(int* out4) const {
+  out4[0] = parallel_ ? Net().world : 1;
+  out4[1] = parallel_ ? Net().rank : 0;
+  out4[2] = fused_ ? 1 : (p2p_allreduce_ ? 2 : 0);
+  out4[3] = obj_ && obj_->IsConstantHessian() && !is_goss_ ? 1 : 0;      // GOSS amplifies hessians [LightGBM goss.hpp GetIsConstHessian -> false]
 }
 
 void Booster::InitTraining() {
@@ -1077,129 +1028,17 @@ void Booster::InitTraining() {
     score_.Upload(train->init_score.data(), train->init_score.size(), stream_);
   }
   // ---- objective set-up
-  class_need_train_.assign(K, true);
-  const_hessian_ = false;
-  if (cfg.objective == "regression") {
-    const_hessian_ = train->weight.empty() && !is_goss_;      // GOSS amplifies hessians [LightGBM goss.hpp GetIsConstHessian -> false]
-  } else if (regvar_kind_) {
-    if (regvar_kind_ >= 3) for (int i = 0; i < n; ++i) if (train->label[i] < 0) Fatal("[" + cfg.objective + "]: at least one target label is negative");
-  } else if (renew_kind_) {
-    const_hessian_ = train->weight.empty() && !is_goss_;
-    if (renew_kind_ == 3) {       // [LightGBM RegressionMAPELOSS::Init] label_weight = 1 / max(1, |label|) (* weight)
-      label_weight_host_.resize(n);
-      for (int i = 0; i < n; ++i) {
-        label_weight_host_[i] = 1.0f / std::max(1.0f, std::fabs(train->label[i]));
-        if (!train->weight.empty()) label_weight_host_[i] *= train->weight[i];
-      }
-      label_weight_.Alloc(n); label_weight_.Upload(label_weight_host_.data(), n, stream_);
-    }
+  obj_->Init(stream_, num_sms_);
+  if (obj_->IsRenewTreeOutput()) {
     // sort buffers of the renewal pass (renew_kernel.cuh)
     rn_keys_a_.Alloc(n); rn_keys_b_.Alloc(n); rn_pos_a_.Alloc(n); rn_pos_b_.Alloc(n); rn_leaf_of_pos_.Alloc(n); rn_leaf_a_.Alloc(n); rn_leaf_b_.Alloc(n);
     rn_res_.Alloc(n); rn_row_.Alloc(n); rn_seg_.Alloc(L + 1); rn_out_.Alloc(2 * static_cast<size_t>(L));
-    if (renew_kind_ == 3 || !train->weight.empty()) rn_cdf_.Alloc(n);
+    if (obj_->RenewWeights()) rn_cdf_.Alloc(n);
     size_t t1 = 0, t2 = 0;
     cub::DeviceRadixSort::SortPairs(nullptr, t1, rn_keys_a_.p, rn_keys_b_.p, rn_pos_a_.p, rn_pos_b_.p, n, 0, 64, stream_);
     cub::DeviceRadixSort::SortPairs(nullptr, t2, rn_leaf_a_.p, rn_leaf_b_.p, rn_pos_b_.p, rn_pos_a_.p, n, 0, 32, stream_);
     rn_tmp_bytes_ = std::max(t1, t2);
     rn_tmp_.Alloc(rn_tmp_bytes_ + 16);
-  } else if (cfg.objective == "binary") {
-    double cnt[2] = {0, 0};
-    for (int i = 0; i < n; ++i) cnt[train->label[i] > 0 ? 1 : 0] += 1;
-    AllReduceHost(cnt, 2, ncclSum, stream_);          // global class counts (R14)
-    binary_need_train_ = !(cnt[0] == 0 || cnt[1] == 0);
-    binary_w_[0] = binary_w_[1] = 1.0;
-    if (cfg.is_unbalance && cnt[0] > 0 && cnt[1] > 0) {
-      if (cnt[1] > cnt[0]) { binary_w_[1] = 1.0; binary_w_[0] = cnt[1] / cnt[0]; }
-      else { binary_w_[1] = cnt[0] / cnt[1]; binary_w_[0] = 1.0; }
-    }
-    binary_w_[1] *= cfg.scale_pos_weight;
-    class_need_train_[0] = binary_need_train_;
-  } else if (cfg.objective == "multiclass") {
-    class_init_probs_.assign(K + 1, 0.0);
-    for (int i = 0; i < n; ++i) {
-      int l = static_cast<int>(train->label[i]);
-      if (l < 0 || l >= K) Fatal("Label must be in [0, " + std::to_string(K) + "), but found " + std::to_string(l) + " in label");
-      double w = train->weight.empty() ? 1.0 : train->weight[i];
-      class_init_probs_[l] += w; class_init_probs_[K] += w;
-    }
-    AllReduceHost(class_init_probs_.data(), K + 1, ncclSum, stream_);
-    for (int k = 0; k < K; ++k) {
-      class_init_probs_[k] /= class_init_probs_[K];
-      class_need_train_[k] = !(std::fabs(class_init_probs_[k]) <= kEps || std::fabs(class_init_probs_[k]) >= 1.0 - kEps);
-    }
-  } else if (is_ova_) {       // [UPSTREAM MulticlassOVA::Init]: one BinaryLogloss::Init per class on (label == k)
-    std::vector<double> cnt(K, 0.0);
-    for (int i = 0; i < n; ++i) {
-      const int l = static_cast<int>(train->label[i]);
-      if (l < 0 || l >= K) Fatal("Label must be in [0, " + std::to_string(K) + "), but found " + std::to_string(l) + " in label");
-      cnt[l] += 1;
-    }
-    double total = n;
-    AllReduceHost(cnt.data(), K, ncclSum, stream_);
-    AllReduceHost(&total, 1, ncclSum, stream_);
-    std::vector<double> cw(2 * static_cast<size_t>(K), 1.0);
-    std::vector<uint8_t> need(K, 1);
-    for (int k = 0; k < K; ++k) {
-      const double pos = cnt[k], neg = total - cnt[k];
-      class_need_train_[k] = !(pos == 0 || neg == 0);
-      need[k] = class_need_train_[k] ? 1 : 0;
-      if (cfg.is_unbalance && pos > 0 && neg > 0) {
-        if (pos > neg) { cw[2 * k + 1] = 1.0; cw[2 * k] = pos / neg; }
-        else { cw[2 * k + 1] = neg / pos; cw[2 * k] = 1.0; }
-      }
-      cw[2 * k + 1] *= cfg.scale_pos_weight;
-    }
-    ova_w_.Alloc(cw.size()); ova_w_.Upload(cw.data(), cw.size(), stream_);
-    ova_need_.Alloc(K); ova_need_.Upload(need.data(), K, stream_);
-    B200_CUDA(cudaStreamSynchronize(stream_));
-  } else if (cfg.objective == "cross_entropy") {      // [UPSTREAM CrossEntropy::Init]
-    for (int i = 0; i < n; ++i)
-      if (!(train->label[i] >= 0.0f && train->label[i] <= 1.0f)) Fatal("[cross_entropy]: does not tolerate label " + std::to_string(train->label[i]) + " outside [0, 1]");
-    if (!train->weight.empty()) {
-      double sw = 0;
-      for (int i = 0; i < n; ++i) { if (train->weight[i] < 0) Fatal("[cross_entropy]: at least one weight is negative"); sw += train->weight[i]; }
-      if (!(sw > 0)) Fatal("[cross_entropy]: sum of weights is zero");
-    }
-  } else if (cfg.objective == "lambdarank") {
-    std::vector<double> lg = cfg.label_gain;
-    if (lg.empty()) { lg.push_back(0.0); for (int i = 1; i < 31; ++i) lg.push_back(static_cast<double>((1 << i) - 1)); }
-    const int nq = static_cast<int>(train->query_boundaries.size()) - 1;
-    std::vector<double> imd(nq);
-    lr_max_q_ = 0;
-    for (int q = 0; q < nq; ++q) {
-      const int s = train->query_boundaries[q], cnt = train->query_boundaries[q + 1] - s;
-      lr_max_q_ = std::max(lr_max_q_, cnt);
-      std::vector<int> label_cnt(lg.size(), 0);
-      for (int i = 0; i < cnt; ++i) {
-        int l = static_cast<int>(train->label[s + i]);
-        if (l < 0 || l >= static_cast<int>(lg.size())) Fatal("Label excel the max range " + std::to_string(lg.size()) + " for lambdarank");
-        ++label_cnt[l];
-      }
-      int top = static_cast<int>(lg.size()) - 1, k = std::min(cfg.lambdarank_truncation_level, cnt);
-      double m = 0;
-      for (int j = 0; j < k; ++j) {
-        while (top > 0 && label_cnt[top] <= 0) --top;
-        m += (1.0 / std::log2(2.0 + j)) * lg[top];      // discount_[j] * label_gain_[top] as [UPSTREAM DCGCalculator::CalMaxDCGAtK]
-        --label_cnt[top];
-      }
-      imd[q] = m > 0.0 ? 1.0 / m : m;
-    }
-    lr_inv_max_dcg_.Alloc(nq); lr_inv_max_dcg_.Upload(imd.data(), nq, stream_);
-    lr_label_gain_.Alloc(lg.size()); lr_label_gain_.Upload(lg.data(), lg.size(), stream_);
-    const size_t bins_n = 1024 * 1024;
-    lr_min_in_ = -50.0 / cfg.sigmoid / 2; lr_max_in_ = 50.0 / cfg.sigmoid / 2;
-    lr_idx_factor_ = bins_n / (lr_max_in_ - lr_min_in_);
-    std::vector<float> tab(bins_n);
-    for (size_t i = 0; i < bins_n; ++i) tab[i] = static_cast<float>(1.0 / (1.0 + std::exp((i / lr_idx_factor_ + lr_min_in_) * cfg.sigmoid)));
-    lr_sig_table_.Alloc(bins_n); lr_sig_table_.Upload(tab.data(), bins_n, stream_);
-    std::vector<double> disc(static_cast<size_t>(std::max(lr_max_q_, 1)) + 1);       // [UPSTREAM DCGCalculator::Init] discount table, host log2
-    for (size_t i = 0; i < disc.size(); ++i) disc[i] = 1.0 / std::log2(2.0 + i);
-    lr_discount_.Alloc(disc.size()); lr_discount_.Upload(disc.data(), disc.size(), stream_);
-    B200_CUDA(cudaStreamSynchronize(stream_));
-    if (cfg.lambdarank_truncation_level < 1 || cfg.lambdarank_truncation_level > 180) Fatal("lambdarank_truncation_level should be in [1, 180]");
-    size_t smem = LambdarankSmem(lr_max_q_, cfg.lambdarank_truncation_level);
-    if (smem > 200 * 1024) Fatal("a query group is too large for the lambdarank kernel");
-    B200_CUDA(cudaFuncSetAttribute(k_grad_lambdarank, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(std::max<size_t>(smem, 1024))));
   }
   if (parallel_) SetupPeerReduce();
   // ColSampler: one draw at init, then one per tree ([UPSTREAM] ColSampler::SetTrainingData / ResetByTree)
@@ -1228,7 +1067,7 @@ void Booster::InitTraining() {
     DevBuf<double> tmp;
     tmp.Alloc(static_cast<size_t>(K) * n); tmp.Zero(stream_);
     for (int k = 0; k < K; ++k) {
-      double init = (cfg.boost_from_average && !has_init_score_) ? ObjectiveInitScore(k) : 0.0;
+      double init = (cfg.boost_from_average && !has_init_score_) ? obj_->BoostFromScore(k) : 0.0;
       if (!(std::fabs(init) > kEps)) init = 0.0;
       rf_init_scores_[k] = init;
       if (init != 0.0) k_add_const<<<num_sms_ * 4, 256, 0, stream_>>>(tmp.p + static_cast<size_t>(k) * n, n, init);
@@ -1442,56 +1281,9 @@ void Booster::ResetFeaturesByTree() {
   feature_used_.Upload(feature_used_host_.data(), train->nf_pad, stream_);
 }
 
-double Booster::ObjectiveInitScore(int k) {
-  const int n = train->num_data;
-  if (cfg.objective == "regression" || regvar_kind_) {
-    double suml = 0, sumw = 0;
-    if (!train->weight.empty()) for (int i = 0; i < n; ++i) { suml += static_cast<double>(train->label[i]) * train->weight[i]; sumw += train->weight[i]; }
-    else { sumw = n; for (int i = 0; i < n; ++i) suml += train->label[i]; }
-    double v = suml / sumw;
-    if (regvar_kind_ >= 3) v = v > 0 ? std::log(v) : -std::numeric_limits<double>::infinity();
-    if (parallel_) { AllReduceHost(&v, 1, ncclSum, stream_); v /= Net().world; }   // GlobalSyncUpByMean (R11)
-    return v;
-  }
-  if (renew_kind_) {
-    const float* y = train->label.data();
-    double v;
-    if (renew_kind_ == 3) v = LabelWeightedPercentile(y, label_weight_host_.data(), n, 0.5);
-    else if (train->weight.empty()) v = LabelPercentile(y, n, renew_alpha_);
-    else v = LabelWeightedPercentile(y, train->weight.data(), n, renew_alpha_);
-    if (parallel_) { AllReduceHost(&v, 1, ncclSum, stream_); v /= Net().world; }   // GlobalSyncUpByMean
-    return v;
-  }
-  if (cfg.objective == "binary") {
-    double s[2] = {0, 0};
-    if (!train->weight.empty()) for (int i = 0; i < n; ++i) { s[0] += (train->label[i] > 0) * static_cast<double>(train->weight[i]); s[1] += train->weight[i]; }
-    else { s[1] = n; for (int i = 0; i < n; ++i) s[0] += (train->label[i] > 0); }
-    AllReduceHost(s, 2, ncclSum, stream_);
-    double pavg = s[0] / s[1];
-    pavg = std::min(pavg, 1.0 - kEps);
-    pavg = std::max(pavg, kEps);
-    return std::log(pavg / (1.0 - pavg)) / cfg.sigmoid;
-  }
-  if (cfg.objective == "multiclass") return std::log(std::max(kEps, class_init_probs_[k]));
-  if (is_ova_ || cfg.objective == "cross_entropy") {      // BinaryLogloss::BoostFromScore on (label == k) / CrossEntropy::BoostFromScore on the label itself
-    double s[2] = {0, 0};
-    for (int i = 0; i < n; ++i) {
-      const double w = train->weight.empty() ? 1.0 : static_cast<double>(train->weight[i]);
-      const double y = is_ova_ ? (static_cast<int>(train->label[i]) == k ? 1.0 : 0.0) : static_cast<double>(train->label[i]);
-      s[0] += y * w; s[1] += w;
-    }
-    AllReduceHost(s, 2, ncclSum, stream_);
-    double pavg = s[0] / s[1];
-    pavg = std::min(pavg, 1.0 - kEps);
-    pavg = std::max(pavg, kEps);
-    return std::log(pavg / (1.0 - pavg)) / (is_ova_ ? cfg.sigmoid : 1.0);
-  }
-  return 0.0;
-}
-
 double Booster::BoostFromAverage(int k) {
   if (model.trees.empty() && !has_init_score_ && cfg.boost_from_average) {
-    double init = ObjectiveInitScore(k);
+    double init = obj_->BoostFromScore(k);
     if (std::fabs(init) > kEps) {
       const int n = train->num_data;
       k_add_const<<<num_sms_ * 4, 256, 0, stream_>>>(score_.p + static_cast<size_t>(k) * n, n, init);
@@ -1506,33 +1298,7 @@ double Booster::BoostFromAverage(int k) {
 void Booster::ComputeGradients() { ComputeGradientsAt(score_.p); }
 void Booster::ComputeGradientsAt(const double* score_p) {
   NvtxRange nvtx("b200gbm:K1/K2 gradients");
-  const int n = train->num_data;
-  const int grid = num_sms_ * 8;
-  const float* w = train->weight.empty() ? nullptr : train->d_weight.p;
-  if (cfg.objective == "regression") {
-    k_grad_l2<<<grid, 256, 0, stream_>>>(score_p, train->d_label.p, w, grad_.p, hess_.p, n);
-  } else if (renew_kind_) {
-    k_grad_percentile<<<grid, 256, 0, stream_>>>(score_p, train->d_label.p, w, renew_kind_ == 3 ? label_weight_.p : nullptr, grad_.p, hess_.p, n, renew_kind_,
-                                                 static_cast<float>(cfg.alpha));
-  } else if (regvar_kind_) {
-    k_grad_regvar<<<grid, 256, 0, stream_>>>(score_p, train->d_label.p, w, grad_.p, hess_.p, n, regvar_kind_, cfg.alpha, cfg.fair_c,
-                                             cfg.poisson_max_delta_step, cfg.tweedie_variance_power);
-  } else if (cfg.objective == "binary") {
-    if (binary_need_train_)
-      k_grad_binary<<<grid, 256, 0, stream_>>>(score_p, train->d_label.p, w, grad_.p, hess_.p, n, cfg.sigmoid, binary_w_[0], binary_w_[1]);
-  } else if (cfg.objective == "multiclass") {
-    k_grad_softmax<<<grid, 256, 0, stream_>>>(score_p, train->d_label.p, w, grad_.p, hess_.p, n, K, static_cast<double>(K) / (K - 1.0));
-  } else if (is_ova_) {
-    k_grad_ova<<<grid, 256, 0, stream_>>>(score_p, train->d_label.p, w, grad_.p, hess_.p, n, K, cfg.sigmoid, ova_w_.p, ova_need_.p);
-  } else if (cfg.objective == "cross_entropy") {
-    k_grad_xent<<<grid, 256, 0, stream_>>>(score_p, train->d_label.p, w, grad_.p, hess_.p, n);
-  } else if (cfg.objective == "lambdarank") {
-    const int nq = static_cast<int>(train->query_boundaries.size()) - 1;
-    size_t smem = std::max<size_t>(LambdarankSmem(lr_max_q_, cfg.lambdarank_truncation_level), 1024);
-    k_grad_lambdarank<<<std::min(nq, num_sms_ * 16), kLrThreads, smem, stream_>>>(
-        score_p, train->d_label.p, w, train->d_qb.p, nq, lr_inv_max_dcg_.p, lr_label_gain_.p, lr_discount_.p, lr_sig_table_.p, 1024 * 1024, lr_min_in_,
-        lr_max_in_, lr_idx_factor_, cfg.sigmoid, cfg.lambdarank_truncation_level, cfg.lambdarank_norm ? 1 : 0, grad_.p, hess_.p, lr_max_q_);
-  }
+  obj_->GetGradients(score_p, grad_.p, hess_.p);
   B200_CUDA(cudaGetLastError());
   timing.launches += 1;
 }
@@ -1545,8 +1311,9 @@ void Booster::RenewTreeOutput(int k, double rf_pred) {
   cudaStream_t s = stream_;
   TreeCtrl* ctrl = ctrl_.p;
   const int egrid = num_sms_ * 8;
-  const bool weighted = renew_kind_ == 3 || !train->weight.empty();
-  const float* wptr = renew_kind_ == 3 ? label_weight_.p : (train->weight.empty() ? nullptr : train->d_weight.p);
+  const float* wptr = obj_->RenewWeights();
+  const bool weighted = wptr != nullptr;
+  const double alpha = obj_->RenewAlpha();
   k_renew_gather<<<egrid, 256, 0, s>>>(ctrl, leaves_.p, idx0_.p, idx1_.p, train->d_label.p, is_rf_ ? nullptr : score_.p + static_cast<size_t>(k) * n, rf_pred,
                                        rn_keys_a_.p, rn_pos_a_.p, rn_res_.p, rn_leaf_of_pos_.p, rn_row_.p);
   size_t tb = rn_tmp_bytes_;
@@ -1561,10 +1328,10 @@ void Booster::RenewTreeOutput(int k, double rf_pred) {
   double* has = rn_out_.p + L;
   const int lgrid = (L + 127) / 128;
   if (!weighted) {
-    k_renew_unweighted<<<lgrid, 128, 0, s>>>(ctrl, rn_seg_.p, rn_pos_a_.p, rn_res_.p, renew_alpha_, out, has);
+    k_renew_unweighted<<<lgrid, 128, 0, s>>>(ctrl, rn_seg_.p, rn_pos_a_.p, rn_res_.p, alpha, out, has);
   } else {
     k_renew_cdf<<<L, 1024, 0, s>>>(ctrl, rn_seg_.p, rn_pos_a_.p, rn_row_.p, wptr, rn_cdf_.p);
-    k_renew_weighted<<<lgrid, 128, 0, s>>>(ctrl, rn_seg_.p, rn_pos_a_.p, rn_res_.p, rn_cdf_.p, renew_kind_ == 3 ? 0.5 : renew_alpha_, out, has);
+    k_renew_weighted<<<lgrid, 128, 0, s>>>(ctrl, rn_seg_.p, rn_pos_a_.p, rn_res_.p, rn_cdf_.p, alpha, out, has);
   }
   if (parallel_) B200_NCCL(ncclAllReduce(out, out, 2 * static_cast<size_t>(L), ncclDouble, ncclSum, Net().comm, s));
   k_renew_apply<<<lgrid, 128, 0, s>>>(ctrl, tree_dev_, out, has, parallel_ ? 1 : 0);
@@ -1636,7 +1403,7 @@ void Booster::LaunchPartition(int grid, int last) {
 
 // One tree: the whole leaf-wise growth is enqueued without a host sync; leaf choice, smaller/larger
 // selection, partition sizes all live in TreeCtrl / LeafState on the device.
-void Booster::TrainOneTree(int k, HostTree* out) {
+void Booster::TrainOneTree(int k, HostTree* out, bool const_hessian) {
   NvtxRange nvtx_tree("b200gbm:tree");
   EnsureColumnCopy();
   const Dataset& d = *train;
@@ -1651,8 +1418,8 @@ void Booster::TrainOneTree(int k, HostTree* out) {
   B200_CUDA(cudaMemsetAsync(&ctrl->absmax_bits[0], 0, 8, s));
   k_absmax<<<egrid, 256, 0, s>>>(g, h, n, ctrl);
   if (parallel_) B200_NCCL(ncclAllReduce(&ctrl->absmax_bits[0], &ctrl->absmax_bits[0], 2, ncclUint32, ncclMax, Net().comm, s));
-  k_set_scale<<<1, 1, 0, s>>>(ctrl, const_hessian_ ? 1 : 0, 1.0);
-  k_quantize<<<egrid, 256, 0, s>>>(g, h, n, qgh_.p, ctrl, const_hessian_ ? 1 : 0, use_bag_ ? in_bag_.p : nullptr, bag_count_);
+  k_set_scale<<<1, 1, 0, s>>>(ctrl, const_hessian ? 1 : 0, 1.0);
+  k_quantize<<<egrid, 256, 0, s>>>(g, h, n, qgh_.p, ctrl, const_hessian ? 1 : 0, use_bag_ ? in_bag_.p : nullptr, bag_count_);
   if (parallel_) B200_NCCL(ncclAllReduce(&ctrl->root_q[0], &ctrl->root_q[0], 3, ncclInt64, ncclSum, Net().comm, s));
   ResetFeaturesByTree();
   if (use_bag_)      // the root leaf is the ascending in-bag row list (SetBaggingData); partitions then ping-pong idx0/idx1 as usual
@@ -1678,7 +1445,7 @@ void Booster::TrainOneTree(int k, HostTree* out) {
     mark();
     // the scratch histogram H is zero here: zeroed at set-up and by every partition kernel after the scan consumed it
     nvtxRangePushA("b200gbm:K4 histogram");
-    if (const_hessian_)
+    if (const_hessian)
       k4_hist_build_ws<3><<<num_sms_, kWsThreads, kWsSmemBytes, s>>>(d.bins.p, d.rows_stride, d.num_tiles, qgh_.p, qord_.p, idx0_.p, idx1_.p, &ctrl->hist_work,
                                                                      reinterpret_cast<unsigned long long*>(H_.p));
     else
@@ -1693,7 +1460,7 @@ void Booster::TrainOneTree(int k, HostTree* out) {
       int units = 0;
       for (const WideMeta& wm : d.wide_host) units += (wm.num_bin + kWideHistSeg - 1) / kWideHistSeg;
       const dim3 wgrid(static_cast<unsigned>(std::max(1, std::min(64, 4 * num_sms_ / std::max(1, units)))), static_cast<unsigned>(d.nw), static_cast<unsigned>(segs));
-      if (const_hessian_)
+      if (const_hessian)
         k4_hist_wide<3><<<wgrid, kWideThreads, 4 * kWideHistSeg * 4, s>>>(d.bins16.p, d.rows_stride, d.wide_meta.p, qgh_.p, qord_.p, idx0_.p, idx1_.p, &ctrl->hist_work,
                                                                          reinterpret_cast<unsigned long long*>(H_.p));
       else
@@ -1737,7 +1504,7 @@ void Booster::TrainOneTree(int k, HostTree* out) {
     mark();
     timing.launches += fused_ ? 4 : 3; timing.hist_launches += 1;
   }
-  if (renew_kind_) RenewTreeOutput(k, is_rf_ ? rf_init_scores_[k] : 0.0);
+  if (obj_->IsRenewTreeOutput()) RenewTreeOutput(k, is_rf_ ? rf_init_scores_[k] : 0.0);
   // rf keeps scores as the running average of (tree + init score) over the iterations [LightGBM rf.hpp MultiplyScore / UpdateScore]
   const double bias = is_rf_ ? rf_init_scores_[k] : 0.0, pre = is_rf_ ? static_cast<double>(iter + num_init_iteration) : 1.0;
   const double post = is_rf_ ? 1.0 / (iter + num_init_iteration + 1) : 1.0;
@@ -1824,7 +1591,7 @@ bool Booster::TrainTrees(const float* custom_g, const float* custom_h) {
   const int n = train->num_data;
   B200_CUDA(cudaEventRecord(ev_a_, s));
   std::vector<double> init_scores(K, 0.0);
-  bool saved_const = const_hessian_;
+  const bool const_hessian = obj_->IsConstantHessian() && !is_goss_ && !custom_g;      // GOSS amplifies hessians; custom ones are arbitrary
   if (is_rf_) {
     if (custom_g) Fatal("RF mode do not support custom objective function, please use built-in objectives.");
     init_scores = rf_init_scores_;
@@ -1835,7 +1602,6 @@ bool Booster::TrainTrees(const float* custom_g, const float* custom_h) {
   } else {
     grad_.Upload(custom_g, static_cast<size_t>(K) * n, s);
     hess_.Upload(custom_h, static_cast<size_t>(K) * n, s);
-    const_hessian_ = false;
   }
   Bagging(iter);
   bool should_continue = is_rf_;        // a random forest never stops early
@@ -1843,13 +1609,13 @@ bool Booster::TrainTrees(const float* custom_g, const float* custom_h) {
     std::unique_ptr<HostTree> t(new HostTree());
     t->Resize(1);
     t->leaf_value[0] = 0;
-    if (class_need_train_[k] && train->nf > 0) TrainOneTree(k, t.get());
+    if (obj_->ClassNeedTrain(k) && train->nf > 0) TrainOneTree(k, t.get(), const_hessian);
     if (t->num_leaves > 1) {
       should_continue = true;
       t->Shrink(shrinkage_);
       if (std::fabs(init_scores[k]) > kEps) t->AddBias(init_scores[k]);
     } else if (static_cast<int>(model.trees.size()) < K) {
-      double output = class_need_train_[k] ? init_scores[k] : ObjectiveInitScore(k);
+      double output = obj_->ClassNeedTrain(k) ? init_scores[k] : obj_->BoostFromScore(k);
       t->MakeConstant(output);
       const double pre = is_rf_ ? static_cast<double>(iter + num_init_iteration) : 1.0, post = is_rf_ ? 1.0 / (iter + num_init_iteration + 1) : 1.0;
       k_scale_add<<<num_sms_ * 4, 256, 0, s>>>(score_.p + static_cast<size_t>(k) * n, n, pre, output, post);
@@ -1864,7 +1630,6 @@ bool Booster::TrainTrees(const float* custom_g, const float* custom_h) {
       B200_CUDA(cudaMemcpyAsync(tree_store_.back()->p, tree_blob_.p, tree_blob_bytes_, cudaMemcpyDeviceToDevice, s));
     }
   }
-  const_hessian_ = saved_const;
   B200_CUDA(cudaEventRecord(ev_b_, s));
   B200_CUDA(cudaEventSynchronize(ev_b_));
   float ms = 0;
@@ -2063,7 +1828,7 @@ std::vector<double> Booster::GetEval(int data_idx) {
   for (auto& m : cfg.metric) {
     const int kind = MetricKindOf(m);
     if (kind >= 0) {
-      MetricParams mp{kind, K, is_ova_ ? 1 : 0, 0, cfg.alpha, cfg.fair_c, cfg.tweedie_variance_power, cfg.sigmoid};
+      MetricParams mp{kind, K, obj_->IsOva() ? 1 : 0, 0, cfg.alpha, cfg.fair_c, cfg.tweedie_variance_power, cfg.sigmoid};
       if ((kind == kMetMultiLogloss || kind == kMetMultiError) && K < 2) Fatal("metric " + m + " needs a multiclass objective");
       k_metric_pointwise<<<grid, kMetricBlock, 0, s>>>(sc.p, d_y, d_w, n, mp, met_partial_.p);
       k_metric_finish<<<1, 32, 0, s>>>(met_partial_.p, grid, 2, met_out_.p);

@@ -47,6 +47,7 @@ void SetThreadDevice(int ordinal);
 void EnsureDevice();            // cudaSetDevice(CurrentDevice()) + fail loudly when no GPU
 void NetworkInit(const char* machines, int local_listen_port, int listen_time_out_sec, int num_machines);
 void NetworkFree();
+void AllReduceHost(double* v, int n, ncclRedOp_t op, cudaStream_t s);      // small host-value collective; no-op without a network
 
 template <typename T>
 struct DevBuf {
@@ -136,6 +137,8 @@ class Dataset {
 };
 
 // ---- booster -----------------------------------------------------------------------------------
+class Objective;       // objective.cuh
+
 struct ValidSet {
   const Dataset* ds = nullptr;
   DevBuf<double> score;   // [K][n]
@@ -162,7 +165,7 @@ class Booster {
   // Returns the number of doubles written to `out` (host).  last_predict_ms = kernel time (CUDA events), incl. H2D for host input.
   int64_t PredictBatch(const void* data, int data_type, int64_t nrow, int ncol, int predict_type, int start_iteration, int num_iteration, double* out);
   double last_predict_ms = 0.0;
-  void GetInfo(int* out4) const { out4[0] = parallel_ ? Net().world : 1; out4[1] = parallel_ ? Net().rank : 0; out4[2] = fused_ ? 1 : (p2p_allreduce_ ? 2 : 0); out4[3] = const_hessian_ ? 1 : 0; }
+  void GetInfo(int* out4) const;
   std::string SaveModelToString(int start_iteration, int num_iteration, int importance_type) const;
   std::string DumpModelJson(int start_iteration, int num_iteration) const;
 
@@ -184,27 +187,17 @@ class Booster {
   void InitTraining();
   void ComputeGradients();
   bool TrainTrees(const float* custom_g, const float* custom_h);
-  void TrainOneTree(int class_id, HostTree* out);
+  void TrainOneTree(int class_id, HostTree* out, bool const_hessian);
   void LaunchPartition(int grid, int last);
   int part_max_blocks_ = 148;
   double BoostFromAverage(int class_id);
-  double ObjectiveInitScore(int class_id);
-  std::string ObjectiveString() const;
 
   int device_ = 0;
   cudaStream_t stream_ = nullptr;
   bool parallel_ = false;
-  bool const_hessian_ = false;
+  std::unique_ptr<Objective> obj_;      // null in a prediction-only booster
   bool has_init_score_ = false;
   double shrinkage_ = 0.1;
-  std::vector<bool> class_need_train_;
-  double binary_w_[2] = {1.0, 1.0};
-  bool binary_need_train_ = true;
-  std::vector<double> class_init_probs_;
-  int regvar_kind_ = 0;                 // 1 huber, 2 fair, 3 poisson, 4 gamma, 5 tweedie
-  bool is_ova_ = false;                 // multiclassova: K independent binary objectives on (label == k)
-  DevBuf<double> ova_w_;                // [K][2] {w_neg, w_pos}
-  DevBuf<uint8_t> ova_need_;            // [K] class has both positives and negatives
   LcgRandom col_rand_{2};               // ColSampler (feature_fraction)
   std::vector<uint8_t> feature_used_host_;
   DevBuf<uint8_t> feature_used_;
@@ -220,10 +213,6 @@ class Booster {
   void Bagging(int it);
   void ComputeGradientsAt(const double* score);
   // percentile objectives: regression_l1 / quantile / mape renew the leaf outputs after the tree is grown (renew_kernel.cuh)
-  int renew_kind_ = 0;                  // 0 none, 1 l1, 2 quantile, 3 mape
-  double renew_alpha_ = 0.5;
-  std::vector<float> label_weight_host_;    // mape: 1 / max(1, |label|) (* weight)
-  DevBuf<float> label_weight_;
   DevBuf<unsigned long long> rn_keys_a_, rn_keys_b_;
   DevBuf<unsigned> rn_pos_a_, rn_pos_b_, rn_leaf_of_pos_, rn_leaf_a_, rn_leaf_b_;
   DevBuf<double> rn_res_, rn_cdf_, rn_out_;      // rn_out_: [2][num_leaves] outputs, has-rows flags
@@ -270,11 +259,6 @@ class Booster {
  private:
   DevBuf<unsigned> part_bits_;
   DevBuf<int> part_chunks_;
-  // lambdarank
-  DevBuf<double> lr_inv_max_dcg_, lr_label_gain_, lr_discount_;
-  DevBuf<float> lr_sig_table_;
-  double lr_min_in_ = -50, lr_max_in_ = 50, lr_idx_factor_ = 0;
-  int lr_max_q_ = 0;
   // fused data-parallel reduce (peer memory over NVLink); falls back to NCCL when peers cannot map each other
   bool fused_ = false;
   bool p2p_allreduce_ = false;          // B200GBM_FUSED_REDUCE=2: the per-split histogram all-reduce is k_allreduce_p2p instead of ncclAllReduce

@@ -1,4 +1,4 @@
-// sm_100a kernels of the b200gbm training engine other than K4 (hist_kernel.cuh).
+// sm_100a kernels of the b200gbm training engine other than K4 (hist_kernel.cuh) and the K1/K2 gradients (objective.cuh).
 // Kernel numbering follows SURVEY.md §2.5.  Everything a tree needs lives in device memory
 // (leaf table, control block, tree arrays) so the host enqueues a whole tree without a sync.
 #pragma once
@@ -180,230 +180,6 @@ k_bin_rows(const T* __restrict__ X, long long nrow, int ncol, int row_major, lon
       }
     }
     bins[(static_cast<size_t>(tile) * rows_stride + row_offset + r) * 32 + lane] = static_cast<uint8_t>(bin);
-  }
-}
-
-// ---------------------------------------------------------------- K1 gradients
-// [UPSTREAM RegressionL2loss::GetGradients]
-__global__ void k_grad_l2(const double* __restrict__ score, const float* __restrict__ label, const float* __restrict__ weight,
-                          float* __restrict__ g, float* __restrict__ h, int n) {
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-    if (weight) { g[i] = static_cast<float>((score[i] - label[i]) * weight[i]); h[i] = weight[i]; }
-    else { g[i] = static_cast<float>(score[i] - label[i]); h[i] = 1.0f; }
-  }
-}
-// [UPSTREAM RegressionHuberLoss / FairLoss / PoissonLoss / GammaLoss / TweedieLoss ::GetGradients]; kind 1..5
-__global__ void k_grad_regvar(const double* __restrict__ score, const float* __restrict__ label, const float* __restrict__ weight,
-                              float* __restrict__ g, float* __restrict__ h, int n, int kind, double alpha, double c, double mds, double rho) {
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-    const double s = score[i], lab = label[i];
-    double gg, hh;
-    if (kind == 1) { const double diff = s - lab; gg = fabs(diff) <= alpha ? diff : d_sign(diff) * alpha; hh = 1.0; }
-    else if (kind == 2) { const double x = s - lab; gg = c * x / (fabs(x) + c); hh = c * c / ((fabs(x) + c) * (fabs(x) + c)); }
-    else if (kind == 3) { gg = exp(s) - lab; hh = exp(s + mds); }
-    else if (kind == 4) { gg = 1.0 - lab * exp(-s); hh = lab * exp(-s); }
-    else { gg = -lab * exp((1 - rho) * s) + exp((2 - rho) * s); hh = -lab * (1 - rho) * exp((1 - rho) * s) + (2 - rho) * exp((2 - rho) * s); }
-    if (weight) { gg *= weight[i]; hh *= weight[i]; }
-    g[i] = static_cast<float>(gg); h[i] = static_cast<float>(hh);
-  }
-}
-// [LightGBM RegressionL1loss / RegressionQuantileloss / RegressionMAPELOSS ::GetGradients]; kind 1 l1, 2 quantile, 3 mape
-__global__ void k_grad_percentile(const double* __restrict__ score, const float* __restrict__ label, const float* __restrict__ weight,
-                                  const float* __restrict__ label_weight, float* __restrict__ g, float* __restrict__ h, int n, int kind, float alpha) {
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-    if (kind == 2) {
-      const float delta = static_cast<float>(score[i] - label[i]);
-      const float gg = delta >= 0 ? (1.0f - alpha) : -alpha;
-      g[i] = weight ? __fmul_rn(gg, weight[i]) : gg;
-    } else {
-      const double diff = score[i] - label[i];
-      const int sgn = (diff > 0.0) - (diff < 0.0);
-      if (kind == 1) g[i] = weight ? static_cast<float>(sgn * static_cast<double>(weight[i])) : static_cast<float>(sgn);
-      else g[i] = static_cast<float>(sgn * static_cast<double>(label_weight[i]));
-    }
-    h[i] = weight ? weight[i] : 1.0f;
-  }
-}
-// [UPSTREAM BinaryLogloss::GetGradients]
-__global__ void k_grad_binary(const double* __restrict__ score, const float* __restrict__ label, const float* __restrict__ weight,
-                              float* __restrict__ g, float* __restrict__ h, int n, double sigmoid, double w_neg, double w_pos) {
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-    const int is_pos = label[i] > 0;
-    const double lab = is_pos ? 1.0 : -1.0;
-    const double lw = is_pos ? w_pos : w_neg;
-    const double response = -lab * sigmoid / (1.0 + exp(lab * sigmoid * score[i]));
-    const double abs_response = fabs(response);
-    double gg = response * lw, hh = abs_response * (sigmoid - abs_response) * lw;
-    if (weight) { gg *= weight[i]; hh *= weight[i]; }
-    g[i] = static_cast<float>(gg); h[i] = static_cast<float>(hh);
-  }
-}
-// [UPSTREAM MulticlassOVA::GetGradients]: class k is a BinaryLogloss on (label == k); cw = per-class {w_neg, w_pos}, need = per-class need_train
-__global__ void k_grad_ova(const double* __restrict__ score, const float* __restrict__ label, const float* __restrict__ weight, float* __restrict__ g,
-                           float* __restrict__ h, int n, int K, double sigmoid, const double* __restrict__ cw, const uint8_t* __restrict__ need) {
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-    const int li = static_cast<int>(label[i]);
-    for (int k = 0; k < K; ++k) {
-      if (!need[k]) continue;
-      const size_t id = static_cast<size_t>(n) * k + i;
-      const int is_pos = li == k;
-      const double lab = is_pos ? 1.0 : -1.0;
-      const double lw = cw[2 * k + is_pos];
-      const double response = -lab * sigmoid / (1.0 + exp(lab * sigmoid * score[id]));
-      const double abs_response = fabs(response);
-      double gg = response * lw, hh = abs_response * (sigmoid - abs_response) * lw;
-      if (weight) { gg *= weight[i]; hh *= weight[i]; }
-      g[id] = static_cast<float>(gg); h[id] = static_cast<float>(hh);
-    }
-  }
-}
-// [UPSTREAM CrossEntropy::GetGradients]: labels are probabilities
-__global__ void k_grad_xent(const double* __restrict__ score, const float* __restrict__ label, const float* __restrict__ weight, float* __restrict__ g,
-                            float* __restrict__ h, int n) {
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-    const double z = 1.0 / (1.0 + exp(-score[i]));
-    double gg = z - label[i], hh = z * (1.0 - z);
-    if (weight) { gg *= weight[i]; hh *= weight[i]; }
-    g[i] = static_cast<float>(gg); h[i] = static_cast<float>(hh);
-  }
-}
-// [UPSTREAM MulticlassSoftmax::GetGradients]; score/g/h are class-major [K][n]
-__global__ void k_grad_softmax(const double* __restrict__ score, const float* __restrict__ label, const float* __restrict__ weight,
-                               float* __restrict__ g, float* __restrict__ h, int n, int K, double factor) {
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-    double wmax = score[i];
-    for (int k = 1; k < K; ++k) wmax = fmax(wmax, score[static_cast<size_t>(n) * k + i]);
-    double wsum = 0;
-    for (int k = 0; k < K; ++k) wsum += exp(score[static_cast<size_t>(n) * k + i] - wmax);
-    const int lab = static_cast<int>(label[i]);
-    const double w = weight ? weight[i] : 1.0;
-    for (int k = 0; k < K; ++k) {
-      double p = exp(score[static_cast<size_t>(n) * k + i] - wmax) / wsum;
-      double gg = (lab == k) ? p - 1.0 : p, hh = factor * p * (1.0 - p);
-      if (weight) { gg *= w; hh *= w; }
-      g[static_cast<size_t>(n) * k + i] = static_cast<float>(gg);
-      h[static_cast<size_t>(n) * k + i] = static_cast<float>(hh);
-    }
-  }
-}
-
-// [UPSTREAM LambdarankNDCG::GetGradientsForOneQuery] — one block per query (K2).
-// Sorting: stable rank by score descending (rank counting out of shared memory; queries are ~100 docs).
-// Pairs (i, j), i < min(truncation, cnt-1), j > i, are evaluated ONCE, tile by tile over j, by all threads (balanced) into a
-// shared-memory matrix M[i][j] = (+-p_lambda, p_hessian) as fp32; then one thread per DOCUMENT adds its entries in the reference's own
-// pair order — for document p: (0,p), (1,p) .. (p-1,p), then (p,p+1) .. (p,cnt-1) — with fp32 adds on a score_t accumulator.  No atomics
-// (shared-memory float atomicAdd is a CAS loop on sm_100a), no double evaluation (the pair math is fp64 with a software division and a
-// table look-up: the first version of this kernel, which evaluated every pair once per side, was FP64-bound at 2.4 ms per 50k queries),
-// and every document's lambda / hessian is the same sequence of fp32 additions as the sequential reference: gradients are reproducible
-// and equal to the oracle's up to the fp64 rounding of the normalisation factor.  discount[] = 1 / log2(2 + pos) is the host-computed
-// table the reference uses (DCGCalculator), not a device log2.
-constexpr int kLrThreads = 128;
-__host__ __device__ inline int lr_tile(int truncation) {          // j-tile width: M = truncation x (tile + 1) float2 within 48 KB
-  int t = (48 * 1024 / 8) / max(truncation, 1) - 1;
-  t = min(t, 128);                 // queries are ~100 documents: one tile, and 20 KB per block keeps 8+ blocks per SM
-  return max(t & ~31, 32);
-}
-__global__ void __launch_bounds__(kLrThreads)
-k_grad_lambdarank(const double* __restrict__ score, const float* __restrict__ label, const float* __restrict__ weight,
-                  const int* __restrict__ qb, int nq, const double* __restrict__ inv_max_dcg, const double* __restrict__ label_gain,
-                  const double* __restrict__ discount, const float* __restrict__ sig_table, int sig_bins, double min_in, double max_in,
-                  double idx_factor, double sigmoid, int truncation, int norm, float* __restrict__ g, float* __restrict__ h, int max_q) {
-  extern __shared__ unsigned char lr_smem[];
-  double* r_score = reinterpret_cast<double*>(lr_smem);                  // [max_q] scores in document order
-  double* s_score = r_score + max_q;                                     // [max_q] scores by sorted position
-  int* s_lab = reinterpret_cast<int*>(s_score + max_q);                  // label by sorted position
-  int* s_orig = s_lab + max_q;                                           // document index by sorted position
-  float* s_lam = reinterpret_cast<float*>(s_orig + max_q);               // accumulators by sorted position
-  float* s_hes = s_lam + max_q;
-  float2* M = reinterpret_cast<float2*>(s_hes + max_q);                  // [truncation][T + 1]; 32 * max_q bytes precede it: 8-byte aligned
-  __shared__ double s_part[kLrThreads];
-  const int T = lr_tile(truncation), TS = T + 1;
-  for (int q = blockIdx.x; q < nq; q += gridDim.x) {
-    const int start = qb[q], cnt = qb[q + 1] - start;
-    __syncthreads();
-    for (int i = threadIdx.x; i < cnt; i += blockDim.x) r_score[i] = score[start + i];
-    __syncthreads();
-    for (int i = threadIdx.x; i < cnt; i += blockDim.x) {
-      const double si = r_score[i];
-      int rank = 0;
-      for (int j = 0; j < cnt; ++j) {
-        const double sj = r_score[j];
-        rank += (sj > si) || (sj == si && j < i);
-      }
-      s_score[rank] = si; s_lab[rank] = static_cast<int>(label[start + i]); s_orig[rank] = i;
-      s_lam[rank] = 0.f; s_hes[rank] = 0.f;
-    }
-    __syncthreads();
-    const double imd = inv_max_dcg[q];
-    const double best_score = s_score[0];
-    int worst_idx = cnt - 1;
-    if (worst_idx > 0 && s_score[worst_idx] == kNegInf) worst_idx -= 1;
-    const double worst_score = s_score[worst_idx];
-    const bool do_div = norm && best_score != worst_score;
-    const int teff = min(truncation, cnt - 1);          // pairs exist for i < teff
-    double local_sum = 0.0;
-    for (int j0 = 0; j0 < cnt; j0 += T) {
-      const int tcnt = min(T, cnt - j0);
-      // ---- phase A: every pair of the tile once
-      for (int e = threadIdx.x; e < teff * tcnt; e += blockDim.x) {
-        const int i = e / tcnt, jj = e - i * tcnt, j = j0 + jj;
-        float2 m = make_float2(0.f, 0.f);
-        if (j > i) {
-          const double sci = s_score[i], scj = s_score[j];
-          const int li = s_lab[i], lj = s_lab[j];
-          if (sci != kNegInf && scj != kNegInf && li != lj) {
-            const bool ih = li > lj;                     // position i holds the higher label
-            const int hr = ih ? i : j, lr = ih ? j : i;
-            const double delta_score = ih ? sci - scj : scj - sci;
-            const double dcg_gap = label_gain[ih ? li : lj] - label_gain[ih ? lj : li];
-            const double paired_discount = fabs(discount[hr] - discount[lr]);
-            double delta = dcg_gap * paired_discount * imd;
-            if (do_div) delta /= (0.01f + fabs(delta_score));
-            double pl;
-            if (delta_score <= min_in) pl = sig_table[0];
-            else if (delta_score >= max_in) pl = sig_table[sig_bins - 1];
-            else pl = sig_table[static_cast<size_t>((delta_score - min_in) * idx_factor)];
-            double ph = pl * (1.0f - pl);
-            pl *= -sigmoid * delta;
-            ph *= sigmoid * sigmoid * delta;
-            local_sum -= 2 * pl;
-            const float fl = static_cast<float>(pl);
-            m = make_float2(ih ? fl : -fl, static_cast<float>(ph));      // lambdas[i] += m.x, lambdas[j] -= m.x (x - y == x + (-y) exactly)
-          }
-        }
-        M[i * TS + jj] = m;
-      }
-      __syncthreads();
-      // ---- phase B: one thread per document, the reference's order of additions
-      for (int p = threadIdx.x; p < cnt; p += blockDim.x) {
-        const bool as_j = p >= j0 && p < j0 + tcnt, as_i = p < teff && p + 1 < j0 + tcnt;
-        if (!as_j && !as_i) continue;
-        float lam = s_lam[p], hes = s_hes[p];
-        if (as_j) {
-          const int ilim = min(p, teff);
-          for (int i = 0; i < ilim; ++i) { const float2 m = M[i * TS + (p - j0)]; lam = __fsub_rn(lam, m.x); hes = __fadd_rn(hes, m.y); }
-        }
-        if (as_i) {
-          for (int j = max(j0, p + 1); j < j0 + tcnt; ++j) { const float2 m = M[p * TS + (j - j0)]; lam = __fadd_rn(lam, m.x); hes = __fadd_rn(hes, m.y); }
-        }
-        s_lam[p] = lam; s_hes[p] = hes;
-      }
-      __syncthreads();
-    }
-    s_part[threadIdx.x] = local_sum;
-    __syncthreads();
-    double sum_lambdas = 0.0;
-    if (norm) for (int t = 0; t < static_cast<int>(blockDim.x); ++t) sum_lambdas += s_part[t];      // fixed order: reproducible
-    double nf = 1.0;
-    const bool do_norm = norm && sum_lambdas > 0;
-    if (do_norm) nf = log2(1 + sum_lambdas) / sum_lambdas;
-    for (int r = threadIdx.x; r < cnt; r += blockDim.x) {
-      float lam = s_lam[r], hes = s_hes[r];
-      if (do_norm) { lam = static_cast<float>(lam * nf); hes = static_cast<float>(hes * nf); }
-      const int o = start + s_orig[r];
-      if (weight) { lam = static_cast<float>(lam * weight[o]); hes = static_cast<float>(hes * weight[o]); }
-      g[o] = lam; h[o] = hes;
-    }
   }
 }
 
