@@ -189,6 +189,9 @@ int B200GBM_DatasetHistogram(DatasetHandle handle, const float* grad, const floa
 int B200GBM_BoosterSetProfile(BoosterHandle handle, int profile_hist);
 int B200GBM_BoosterGetTiming(BoosterHandle handle, double* out6, int reset);
 int B200GBM_BoosterGetScores(BoosterHandle handle, int data_idx, double* out);    /* raw scores, class-major */
+/* for tests: the objective's gradients and hessians at the current training scores (the init_score before the first iteration),
+ * class-major [num_class][num_data] fp32; classes the objective does not train read 0.  Changes neither the model nor the scores. */
+int B200GBM_BoosterGetGradients(BoosterHandle handle, float* out_grad, float* out_hess);
 /* batched GPU prediction (SURVEY §8f-2): row-major matrix on the host or the device, predict_type NORMAL / RAW_SCORE / LEAF_INDEX /
  * CONTRIB (TreeSHAP, [nrow][num_class][num_feature+1]); values equal LGBM_BoosterPredictForMatSingle row by row (raw scores and leaf
  * indices bit for bit, contributions to 1e-12); out_result is a host buffer sized by LGBM_BoosterCalcNumPredict; elapsed_ms (may be

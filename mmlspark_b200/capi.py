@@ -438,6 +438,17 @@ class Booster:
         check(load().B200GBM_BoosterGetScores(self.handle, C.c_int(data_idx), _ptr(out)))
         return out
 
+    def get_gradients(self):
+        """For tests: (grad, hess), float32 arrays of K * num_data (class-major), the objective's gradients at the current training
+        scores, which before the first iteration are the training set's init_score.  Classes the objective does not train read 0.
+        Training is not affected: the model and the scores stay as they are."""
+        n = C.c_int64(0)
+        check(load().LGBM_BoosterGetNumPredict(self.handle, C.c_int(0), C.byref(n)))
+        g = np.zeros(n.value, dtype=np.float32)
+        h = np.zeros(n.value, dtype=np.float32)
+        check(load().B200GBM_BoosterGetGradients(self.handle, _ptr(g), _ptr(h)))
+        return g, h
+
     def free(self):
         if self.handle:
             check(load().LGBM_BoosterFree(self.handle))

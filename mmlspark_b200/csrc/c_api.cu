@@ -607,4 +607,9 @@ int B200GBM_BoosterGetScores(BoosterHandle handle, int data_idx, double* out) {
   BS(handle)->GetRawScores(data_idx, out);
   API_END();
 }
+int B200GBM_BoosterGetGradients(BoosterHandle handle, float* out_grad, float* out_hess) {
+  API_BEGIN();
+  BS(handle)->GetGradients(out_grad, out_hess);
+  API_END();
+}
 }  // extern "C"

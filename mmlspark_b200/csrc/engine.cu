@@ -893,6 +893,7 @@ Booster::Booster(const Dataset* tr, const char* params) : train(tr) {
   if (cfg.num_leaves < 2) Fatal("num_leaves should be >= 2");
   ValidateMetrics();      // an unknown metric must fail LGBM_BoosterCreate, not the first LGBM_BoosterGetEval inside the training loop
   obj_->CheckData();
+  CheckMetricLabels(train, cfg);
   K = obj_->NumModelPerIteration();
   parallel_ = Net().active && Net().world > 1;
   cfg.num_machines = parallel_ ? Net().world : 1;
@@ -1654,10 +1655,15 @@ bool Booster::UpdateOneIterCustom(const float* grad, const float* hess) { return
 void Booster::ResetParameter(const char* params) {
   Config nc;
   nc.Parse(params);
-  for (auto& kv : nc.raw) cfg.raw[kv.first] = kv.second;
-  int keep_machines = cfg.num_machines;
-  cfg.Refresh();
-  cfg.num_machines = keep_machines;
+  Config next = cfg;
+  for (auto& kv : nc.raw) next.raw[kv.first] = kv.second;
+  next.Refresh();
+  next.num_machines = cfg.num_machines;
+  if (train) {      // checked before the change is applied: a refused reset leaves the booster as it was
+    CheckMetricLabels(train, next);
+    for (auto* v : valids_) CheckMetricLabels(v->ds, next);
+  }
+  cfg = next;       // in place: the objective keeps a reference to cfg
   shrinkage_ = is_rf_ ? 1.0 : cfg.learning_rate;
   if (is_dart_) { drop_rand_ = LcgRandom(cfg.drop_seed); sum_weight_ = 0.0; }      // [LightGBM dart.hpp DART::ResetConfig]
   sp_.l1 = cfg.lambda_l1; sp_.l2 = cfg.lambda_l2; sp_.max_delta_step = cfg.max_delta_step; sp_.min_gain_to_split = cfg.min_gain_to_split;
@@ -1668,6 +1674,7 @@ void Booster::AddValidData(const Dataset* valid) {
   EnsureDevice();
   if (!train) Fatal("cannot add validation data to a prediction-only booster");
   if (valid->nf != train->nf) Fatal("validation data must be created with reference=train");
+  CheckMetricLabels(valid, cfg);
   ValidSet* v = new ValidSet();
   v->ds = valid;
   v->score.Alloc(static_cast<size_t>(K) * valid->num_data);
@@ -1792,6 +1799,10 @@ static int MetricKindOf(const std::string& m) {
   auto it = kinds.find(m);
   return it == kinds.end() ? -1 : it->second;
 }
+// [LightGBM NDCGMetric::Init -> DCGCalculator::CheckLabel]: k_metric_rank indexes label_gain with the labels of every evaluated set
+void Booster::CheckMetricLabels(const Dataset* ds, const Config& c) const {
+  if (std::find(c.metric.begin(), c.metric.end(), "ndcg") != c.metric.end()) CheckRankLabels(ds->label, RankLabelGain(c).size());
+}
 void Booster::ValidateMetrics() const {
   for (auto& m : cfg.metric)
     if (MetricKindOf(m) < 0 && m != "auc" && m != "ndcg" && m != "map") Fatal("Unknown metric type name: " + m);
@@ -1869,8 +1880,7 @@ std::vector<double> Booster::GetEval(int data_idx) {
       if (!rank_done) {
         const int nq = static_cast<int>(ds->query_boundaries.size()) - 1;
         if (nq <= 0) Fatal("The " + std::string(m == "ndcg" ? "NDCG" : "MAP") + " metric requires query information");
-        std::vector<double> lg = cfg.label_gain;
-        if (lg.empty()) { lg.push_back(0.0); for (int i = 1; i < 31; ++i) lg.push_back(static_cast<double>((1 << i) - 1)); }
+        const std::vector<double> lg = RankLabelGain(cfg);
         int max_q = 1;
         for (int q = 0; q < nq; ++q) max_q = std::max(max_q, ds->query_boundaries[q + 1] - ds->query_boundaries[q]);
         std::vector<double> disc(static_cast<size_t>(max_q) + 1);
@@ -1885,7 +1895,7 @@ std::vector<double> Booster::GetEval(int data_idx) {
         for (int e = 0; e < rp.nk; ++e) rp.ks[e] = ks[e];
         rp.want_ndcg = std::find(cfg.metric.begin(), cfg.metric.end(), "ndcg") != cfg.metric.end();
         rp.want_map = std::find(cfg.metric.begin(), cfg.metric.end(), "map") != cfg.metric.end();
-        const size_t smem = static_cast<size_t>(max_q) * (8 + 4 + 4);
+        const size_t smem = RankMetricSmem(max_q, static_cast<int>(lg.size()));
         if (smem > 200 * 1024) Fatal("a query group is too large for the ranking metric kernel");
         B200_CUDA(cudaFuncSetAttribute(k_metric_rank, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(std::max<size_t>(smem, 1024))));
         const int rgrid = std::max(1, std::min(nq, num_sms_ * 8));
@@ -1909,6 +1919,21 @@ std::vector<double> Booster::GetEval(int data_idx) {
     }
   }
   return out;
+}
+
+// Gradients and hessians of the objective at the current training scores, into scratch buffers: grad_ / hess_ (which random
+// forest reuses across iterations) and the timing counters are left alone, so calling this changes nothing the training sees
+void Booster::GetGradients(float* out_g, float* out_h) {
+  if (!train || !obj_) Fatal("this booster was loaded from a model string: it has no objective to take gradients of");
+  EnsureDevice();
+  const size_t len = static_cast<size_t>(K) * train->num_data;
+  DevBuf<float> g, h;
+  g.Alloc(len); h.Alloc(len);
+  g.Zero(stream_); h.Zero(stream_);      // classes the objective skips stay 0
+  obj_->GetGradients(score_.p, g.p, h.p);
+  B200_CUDA(cudaGetLastError());
+  g.Download(out_g, len, stream_); h.Download(out_h, len, stream_);
+  B200_CUDA(cudaStreamSynchronize(stream_));
 }
 
 void Booster::GetRawScores(int data_idx, double* out) {

@@ -158,9 +158,11 @@ class Booster {
   std::vector<std::string> EvalNames() const;
   std::vector<double> GetEval(int data_idx);
   void ValidateMetrics() const;
+  void CheckMetricLabels(const Dataset* ds, const Config& c) const;      // ndcg: labels index label_gain
   void GetPredict(int data_idx, int64_t* out_len, double* out);
   int64_t NumPredict(int data_idx) const;
   void GetRawScores(int data_idx, double* out);
+  void GetGradients(float* out_g, float* out_h);         // [K][n] at the current training scores (a test hook)
   // batched GPU prediction over a row-major matrix (host or device pointer); predict_type 0 normal, 1 raw, 2 leaf index.
   // Returns the number of doubles written to `out` (host).  last_predict_ms = kernel time (CUDA events), incl. H2D for host input.
   int64_t PredictBatch(const void* data, int data_type, int64_t nrow, int ncol, int predict_type, int start_iteration, int num_iteration, double* out);

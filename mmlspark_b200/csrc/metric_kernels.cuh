@@ -157,14 +157,19 @@ k_auc_terms(const unsigned long long* __restrict__ keys, const int* __restrict__
 // out partial[q_block][2 * nk]: ndcg sums then map sums for the nk cut-offs (ks ascending as the reference sorts eval_at)
 constexpr int kMaxEvalAt = 16;
 struct RankEvalParams { int nk; int ks[kMaxEvalAt]; int want_ndcg, want_map; };
+// dynamic shared memory of k_metric_rank: score, sorted label, label and relevance flag per document, plus the label histogram
+inline size_t RankMetricSmem(int max_q, int num_gain) {
+  return static_cast<size_t>(max_q) * (8 + 4 + 4 + 1) + static_cast<size_t>(num_gain) * 4;
+}
 __global__ void __launch_bounds__(128)
 k_metric_rank(const double* __restrict__ score, const float* __restrict__ label, const int* __restrict__ qb, int nq, const double* __restrict__ label_gain,
               int num_gain, const double* __restrict__ discount, RankEvalParams rp, int max_q, double* __restrict__ partial) {
-  extern __shared__ unsigned char rk_smem[];
+  extern __shared__ unsigned char rk_smem[];                     // RankMetricSmem(max_q, num_gain) bytes
   double* r_score = reinterpret_cast<double*>(rk_smem);          // [max_q] document order
-  int* s_lab = reinterpret_cast<int*>(r_score + max_q);          // [max_q] label by sorted position
+  int* s_lab = reinterpret_cast<int*>(r_score + max_q);          // [max_q] label by sorted position (ndcg: an index of label_gain)
   float* r_lab = reinterpret_cast<float*>(s_lab + max_q);        // [max_q] label in document order
-  __shared__ int s_cnt[64];                                      // label value histogram (label_gain has <= 31 entries by default)
+  int* s_cnt = reinterpret_cast<int*>(r_lab + max_q);            // [num_gain] label value histogram
+  unsigned char* s_rel = reinterpret_cast<unsigned char*>(s_cnt + num_gain);     // [max_q] relevant for MAP (label > 0.5) by sorted position
   double acc[2 * kMaxEvalAt];
   for (int k = 0; k < 2 * kMaxEvalAt; ++k) acc[k] = 0.0;
   const long long per = (static_cast<long long>(nq) + gridDim.x - 1) / gridDim.x;
@@ -172,7 +177,7 @@ k_metric_rank(const double* __restrict__ score, const float* __restrict__ label,
   for (long long q = q0; q < q1; ++q) {
     const int start = qb[q], cnt = qb[q + 1] - start;
     __syncthreads();
-    if (threadIdx.x < 64) s_cnt[threadIdx.x] = 0;
+    for (int v = threadIdx.x; v < num_gain; v += blockDim.x) s_cnt[v] = 0;
     for (int i = threadIdx.x; i < cnt; i += blockDim.x) { r_score[i] = score[start + i]; r_lab[i] = label[start + i]; }
     __syncthreads();
     for (int i = threadIdx.x; i < cnt; i += blockDim.x) {
@@ -180,26 +185,25 @@ k_metric_rank(const double* __restrict__ score, const float* __restrict__ label,
       int rank = 0;
       for (int j = 0; j < cnt; ++j) { const double sj = r_score[j]; rank += (sj > si) || (sj == si && j < i); }
       const int li = static_cast<int>(r_lab[i]);
-      s_lab[rank] = r_lab[i] > 0.5f ? (li | 0x40000000) : li;       // bit 30: "relevant" for MAP (label > 0.5)
-      if (li >= 0 && li < 64) atomicAdd(&s_cnt[li], 1);
+      s_lab[rank] = li;
+      s_rel[rank] = r_lab[i] > 0.5f;
+      if (li >= 0 && li < num_gain) atomicAdd(&s_cnt[li], 1);      // ndcg labels are checked on the host; map-only labels may be anything
     }
     __syncthreads();
     if (threadIdx.x == 0) {
       if (rp.want_ndcg) {
-        // [UPSTREAM DCGCalculator::CalMaxDCG] then CalDCG, both sequential in position order
+        // [UPSTREAM DCGCalculator::CalMaxDCG] then CalDCG, both sequential in position order; the walk consumes s_cnt (reset per query)
         double maxdcg[kMaxEvalAt];
         {
           int top = num_gain - 1, left = 0;
           double cur = 0;
-          int lc[64];
-          for (int v = 0; v < 64; ++v) lc[v] = s_cnt[v];
           for (int e = 0; e < rp.nk; ++e) {
             const int ck = min(rp.ks[e], cnt);
             for (int j = left; j < ck; ++j) {
-              while (top > 0 && lc[top] <= 0) --top;
+              while (top > 0 && s_cnt[top] <= 0) --top;
               if (top < 0) break;
               cur += discount[j] * label_gain[top];
-              --lc[top];
+              --s_cnt[top];
             }
             maxdcg[e] = cur;
             left = ck;
@@ -212,7 +216,7 @@ k_metric_rank(const double* __restrict__ score, const float* __restrict__ label,
           int left = 0;
           for (int e = 0; e < rp.nk; ++e) {
             const int ck = min(rp.ks[e], cnt);
-            for (int j = left; j < ck; ++j) cur += label_gain[s_lab[j] & 0x3fffffff] * discount[j];
+            for (int j = left; j < ck; ++j) cur += label_gain[s_lab[j]] * discount[j];
             acc[e] += cur * (1.0 / maxdcg[e]);
             left = ck;
           }
@@ -221,13 +225,13 @@ k_metric_rank(const double* __restrict__ score, const float* __restrict__ label,
       if (rp.want_map) {
         // [UPSTREAM MapMetric::CalMapAtK]
         int npos = 0;
-        for (int j = 0; j < cnt; ++j) npos += (s_lab[j] >> 30) & 1;
+        for (int j = 0; j < cnt; ++j) npos += s_rel[j];
         int num_hit = 0, left = 0;
         double sum_ap = 0;
         for (int e = 0; e < rp.nk; ++e) {
           const int ck = min(rp.ks[e], cnt);
           for (int j = left; j < ck; ++j)
-            if ((s_lab[j] >> 30) & 1) { ++num_hit; sum_ap += num_hit / (j + 1.0f); }
+            if (s_rel[j]) { ++num_hit; sum_ap += num_hit / (j + 1.0f); }
           acc[kMaxEvalAt + e] += npos > 0 ? sum_ap / min(npos, ck) : 1.0;
           left = ck;
         }

@@ -278,6 +278,24 @@ static float LabelWeightedPercentile(const float* y, const float* w, int cnt, do
   return v2;
 }
 
+// ---- ranking labels (lambdarank objective, ndcg metric)
+// label_gain, or LightGBM's default 2^i - 1 for the labels 0..30
+static std::vector<double> RankLabelGain(const Config& cfg) {
+  std::vector<double> lg = cfg.label_gain;
+  if (lg.empty()) { lg.push_back(0.0); for (int i = 1; i < 31; ++i) lg.push_back(static_cast<double>((1 << i) - 1)); }
+  return lg;
+}
+// [LightGBM DCGCalculator::CheckLabel] a ranking label indexes label_gain: an integer in [0, num_gain)
+static void CheckRankLabels(const std::vector<float>& label, size_t num_gain) {
+  for (const float l : label) {
+    if (std::fabs(l - static_cast<float>(static_cast<int>(l))) > 1e-15f)
+      Fatal("label should be int type (met " + std::to_string(l) + ") for ranking task,\nfor the gain of label, please set the label_gain parameter");
+    if (!(l >= 0)) Fatal("Label should be non-negative (met " + std::to_string(l) + ") for ranking task");
+    if (static_cast<size_t>(l) >= num_gain)
+      Fatal("Label " + std::to_string(static_cast<size_t>(l)) + " is not less than the number of label mappings (" + std::to_string(num_gain) + ")");
+  }
+}
+
 // dynamic shared memory of k_grad_lambdarank: per-document arrays + the pair matrix of one j-tile
 static size_t LambdarankSmem(int max_q, int truncation) {
   return static_cast<size_t>(max_q) * (8 + 8 + 4 + 4 + 4 + 4) + 8 + static_cast<size_t>(truncation) * (lr_tile(truncation) + 1) * 8;
@@ -411,8 +429,8 @@ class Objective {
         }
         break;
       case kLambdarank: {
-        std::vector<double> lg = cfg_.label_gain;
-        if (lg.empty()) { lg.push_back(0.0); for (int i = 1; i < 31; ++i) lg.push_back(static_cast<double>((1 << i) - 1)); }
+        const std::vector<double> lg = RankLabelGain(cfg_);
+        CheckRankLabels(train->label, lg.size());
         const int nq = static_cast<int>(train->query_boundaries.size()) - 1;
         std::vector<double> imd(nq);
         lr_max_q_ = 0;
@@ -420,11 +438,7 @@ class Objective {
           const int s = train->query_boundaries[q], cnt = train->query_boundaries[q + 1] - s;
           lr_max_q_ = std::max(lr_max_q_, cnt);
           std::vector<int> label_cnt(lg.size(), 0);
-          for (int i = 0; i < cnt; ++i) {
-            int l = static_cast<int>(train->label[s + i]);
-            if (l < 0 || l >= static_cast<int>(lg.size())) Fatal("Label excel the max range " + std::to_string(lg.size()) + " for lambdarank");
-            ++label_cnt[l];
-          }
+          for (int i = 0; i < cnt; ++i) ++label_cnt[static_cast<int>(train->label[s + i])];
           int top = static_cast<int>(lg.size()) - 1, k = std::min(cfg_.lambdarank_truncation_level, cnt);
           double m = 0;
           for (int j = 0; j < k; ++j) {

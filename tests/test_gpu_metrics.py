@@ -148,6 +148,100 @@ def test_ranking_metrics_ndcg_and_map(built):
         np.testing.assert_allclose(got[4:], mp, rtol=1e-6)          # [UPSTREAM] accumulates num_hit / (j + 1.0f) in float
 
 
+def _rank_case(rng, max_label):
+    """single-document queries, short ones and one 1000-document query full of tied scores; a validation set of whole queries"""
+    sizes = np.concatenate([np.ones(40, dtype=np.int32), rng.integers(2, 60, 300).astype(np.int32), [1000]]).astype(np.int32)
+    rng.shuffle(sizes)
+    n = int(sizes.sum())
+    X = np.round(rng.standard_normal((n, 5)), 1)
+    y = np.clip(np.round((X[:, 0] + 0.7 * rng.standard_normal(n) + 1.0) * max_label / 4), 0, max_label).astype(np.float32)
+    cut = int(np.searchsorted(np.cumsum(sizes), n // 2, side="right"))
+    return X, y, sizes, cut
+
+
+EVAL_AT_16 = [1, 2, 3, 4, 5, 6, 7, 8, 10, 12, 15, 20, 30, 50, 100, 2000]      # 2000: more than any query holds
+
+
+@pytest.mark.parametrize("num_gain", [31, 40, 100])
+def test_ranking_metrics_long_label_gain(built, num_gain):
+    """k_metric_rank sizes its label histogram from label_gain: with 40 and 100 gains the labels above 63 count towards the max DCG"""
+    rng = np.random.default_rng(num_gain)
+    X, y, sizes, cut = _rank_case(rng, num_gain - 1)
+    gain = _rank_gain(num_gain)
+    nv = int(sizes[:cut].sum())
+    lg = "" if num_gain == 31 else " label_gain=" + ",".join(repr(float(v)) for v in gain)
+    params = "objective=lambdarank metric=ndcg,map eval_at=%s min_data_in_leaf=5%s" % (",".join(map(str, EVAL_AT_16)), lg)
+    b, _, _ = _fit(X, y, params, X[:nv], y[:nv], group=sizes, gv=sizes[:cut], iters=3)
+    assert b.eval_names() == ["ndcg@%d" % k for k in EVAL_AT_16] + ["map@%d" % k for k in EVAL_AT_16]
+    assert y.max() == num_gain - 1
+    for idx, (nn, sz) in enumerate(((len(y), sizes), (nv, sizes[:cut]))):
+        s = b.get_scores(idx)
+        nd, mp = _rank_metrics(s, y[:nn], sz, EVAL_AT_16, gain)
+        got = b.get_eval(idx)
+        np.testing.assert_allclose(got[:16], nd, rtol=1e-10)
+        np.testing.assert_allclose(got[16:], mp, rtol=1e-6)
+
+
+def _rank_gain(num_gain):
+    if num_gain == 31:
+        return np.array([0.0] + [float((1 << i) - 1) for i in range(1, 31)])
+    return np.round(np.arange(num_gain, dtype=np.float64) ** 1.7, 4)
+
+
+def test_map_negative_labels_are_not_relevant(built):
+    """MAP counts label > 0.5 as relevant: -1 is not"""
+    rng = np.random.default_rng(14)
+    sizes = rng.integers(1, 40, 400).astype(np.int32)
+    n = int(sizes.sum())
+    X = np.round(rng.standard_normal((n, 5)), 1)
+    y = rng.choice(np.array([-1, 0, 1, 2], dtype=np.float32), n, p=[0.4, 0.3, 0.2, 0.1])
+    b, _, _ = _fit(X, y, "objective=regression metric=map eval_at=1,3,10,50", group=sizes, iters=2)
+    nd, mp = _rank_metrics(b.get_scores(0), y, sizes, [1, 3, 10, 50], np.zeros(3))
+    np.testing.assert_allclose(b.get_eval(0), mp, rtol=1e-6)
+
+
+def test_ndcg_label_checks(built):
+    """[LightGBM DCGCalculator::CheckLabel] on every dataset the ndcg metric evaluates: labels are integers in [0, label_gain.size())"""
+    from mmlspark_b200 import capi
+    rng = np.random.default_rng(15)
+    n = 2000
+    X = rng.standard_normal((n, 4))
+    group = np.full(n // 20, 20, dtype=np.int32)
+    y = rng.integers(0, 5, n).astype(np.float32)
+
+    def train_set(labels):
+        return capi.Dataset.from_mat(X, DS_PARAMS).set_field("label", labels).set_field("group", group)
+
+    frac = y.copy()
+    frac[17] = 1.5
+    with pytest.raises(capi.LightGBMError, match="label should be int type"):
+        capi.Booster(train_set(frac), BASE + "objective=regression metric=ndcg")
+    with pytest.raises(capi.LightGBMError, match="label should be int type"):
+        capi.Booster(train_set(frac), BASE + "objective=lambdarank")
+    neg = y.copy()
+    neg[3] = -1
+    with pytest.raises(capi.LightGBMError, match="Label should be non-negative"):
+        capi.Booster(train_set(neg), BASE + "objective=regression metric=ndcg")
+    big = y.copy()
+    big[9] = 40
+    with pytest.raises(capi.LightGBMError, match=r"Label 40 is not less than the number of label mappings \(31\)"):
+        capi.Booster(train_set(big), BASE + "objective=regression metric=ndcg")
+    # a validation set whose labels fall outside label_gain is refused when it is added
+    ds = train_set(y)
+    b = capi.Booster(ds, BASE + "objective=lambdarank metric=ndcg label_gain=0,1,3,7,15")
+    dv = capi.Dataset.from_mat(X, DS_PARAMS, reference=ds).set_field("label", np.where(np.arange(n) == 5, 5, y).astype(np.float32))
+    dv.set_field("group", group)
+    with pytest.raises(capi.LightGBMError, match=r"Label 5 is not less than the number of label mappings \(5\)"):
+        b.add_valid(dv)
+    # ... and so is a reset that shortens label_gain below the labels of a dataset already added
+    b2 = capi.Booster(train_set(y), BASE + "objective=regression metric=l2")
+    with pytest.raises(capi.LightGBMError, match=r"Label [34] is not less than the number of label mappings \(3\)"):
+        b2.reset_parameter("metric=ndcg label_gain=0,1,3")
+    assert b2.eval_names() == ["l2"] and len(b2.get_eval(0)) == 1              # the refused reset left the booster as it was
+    # map alone does not index label_gain: negative and large labels are fine
+    capi.Booster(train_set(np.where(np.arange(n) % 7 == 0, -1, 70).astype(np.float32)), BASE + "objective=regression metric=map").get_eval(0)
+
+
 def test_unknown_metric_fails_at_booster_create(built):
     from mmlspark_b200 import capi
     rng = np.random.default_rng(5)
